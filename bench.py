@@ -2,7 +2,7 @@
 """bench.py — throughput of the B200 AV1 reconstruction + post-filter back end (BASELINE.json metric:
 Mpixels/s recon+postfilter @ 4K).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic records, per GPU.
 
@@ -22,6 +22,11 @@ row it reads (dav1d's check_tile rule; dav1d_b200/shard.py). Inside the timed re
 
 --impl reference times dav1d's own C functions (oracle/_ref, unmodified reference sources, HAVE_ASM=0:
 no nasm in this image) on the host cores: one frame per thread (dav1d's frame threading), all cores.
+
+--dump-outputs DIR writes what the timed path computed in its last timed step (the pictures a caller of that path
+receives) as DIR/<name>.npy in float32, so that two builds can be compared output for output: the inputs are seeded and
+the number of frames decoded before it is fixed by the arguments. Above 64 MB in all, every array is cut down to the
+same seeded sample of its elements.
 """
 import os as _os
 # up to 32 hardware work queues, so that the frames in flight (one stream each) really run side by side: with the
@@ -413,7 +418,7 @@ def run_stream(args):
         tus = build()
     px = W["W"] * W["H"] * W["frames"]
     stream.decode_stream.capacity = (W["W"] * W["H"] * 3 // 2) * (2 if W["bpc"] > 8 else 1) * W["frames"] + (1 << 20)
-    steps = min(args.steps, 10)
+    steps = args.steps
     wl = "%s: %s; %d dav1d threads, %d frames in flight" % (args.workload, W["desc"], nthr, mfd)
     if args.impl == "reference":
         if rank != 0:
@@ -456,6 +461,8 @@ def run_stream(args):
     dt = time.perf_counter() - t0
     sampler.stop()
     st = dec.stats()
+    if args.dump_outputs and rank == 0:            # every picture of the last decode, packed plane after plane
+        dump_outputs(args.dump_outputs, {"pictures": out.view(np.uint16) if W["bpc"] > 8 else out})
     if world > 1:
         tt = torch.tensor([dt], device="cuda", dtype=torch.float64)
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -591,6 +598,12 @@ def run_ours_frame(args):
     ev_end.record()
     sync_all()
     launches = lib.b200_launch_count() - launches0
+    if args.dump_outputs and rank == 0:            # the displayed pictures of the frames of the last timed step
+        last = range(nsets) if fps > 1 else [(args.steps - 1) % nsets]
+        arrays = {}
+        for k in last:
+            arrays.update(picture_arrays("picture%d_" % k if fps > 1 else "picture_", Ss[k], fbs[k].output()))
+        dump_outputs(args.dump_outputs, arrays)
     total_ms = ev[0].elapsed_time(ev_end)
     t = torch.tensor([total_ms], device="cuda")
     if world > 1:
@@ -681,16 +694,27 @@ def run_ours_frame(args):
         dist.destroy_process_group()
 
 
-def planes_differ(S, a, b):
-    """first (plane, row) where the visible area of two pictures of frame S differs, or None"""
+def picture_planes(S, pic):
+    """the visible area of each plane of a picture of frame S, as 2-D views"""
     ssh, ssv = [0, S["ss_hor"], S["ss_hor"]], [0, S["ss_ver"], S["ss_ver"]]
+    out = []
     for pl in range(3):
         h, w = (S["H"] + ssv[pl]) >> ssv[pl], (S["W"] + ssh[pl]) >> ssh[pl]
         o, st = S["off"][pl], S["stride"][pl]
-        A = a[o:o + h * st].reshape(h, st)[:, :w]; B = b[o:o + h * st].reshape(h, st)[:, :w]
+        out.append(pic[o:o + h * st].reshape(h, st)[:, :w])
+    return out
+
+
+def planes_differ(S, a, b):
+    """first (plane, row) where the visible area of two pictures of frame S differs, or None"""
+    for pl, (A, B) in enumerate(zip(picture_planes(S, a), picture_planes(S, b))):
         if not np.array_equal(A, B):
             return pl, int(np.where((A != B).any(axis=1))[0][0])
     return None
+
+
+def picture_arrays(prefix, S, pic):
+    return {"%s%s" % (prefix, n): p for n, p in zip(("y", "u", "v"), picture_planes(S, pic))}
 
 
 def dev_to_numpy(lib, ptr, like):
@@ -783,18 +807,10 @@ def run_ours_gop(args):
         for _ in range(nframes):
             pipe.submit()
 
+    # every set runs twice before timing: buffers touched, and with graphs each set's schedule captured (on its 2nd frame)
+    args.warmup = max(args.warmup, 2 * nsets)
     block(args.warmup)
     sync_all()
-    # inner repetitions: the timed region lasts at least ~0.6 s whatever --steps is (clock samples, launch noise)
-    t0 = time.perf_counter()
-    block(args.steps)
-    sync_all()
-    est = time.perf_counter() - t0
-    reps = max(1, int(np.ceil(float(os.environ.get("B200_MIN_TIMED_S", "0.6")) / max(est, 1e-4))))
-    if world > 1:
-        tr = torch.tensor([reps], device="cuda")
-        dist.all_reduce(tr, op=dist.ReduceOp.MAX)
-        reps = int(tr.item())
     sampler = ClockSampler(local)
     sampler.start()
     time.sleep(0.15)
@@ -805,7 +821,7 @@ def run_ours_gop(args):
     ev0.record(main)
     for t in tstreams:
         t.wait_stream(main)             # the timed region starts on every stream after ev0
-    block(args.steps * reps)
+    block(args.steps)
     for t in tstreams:
         main.wait_stream(t)             # ... and ends when every stream (incl. the puts) has drained
     ev1.record(main)
@@ -815,9 +831,12 @@ def run_ours_gop(args):
     t = torch.tensor([ev0.elapsed_time(ev1)], device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
-    ms_per_step = float(t.item()) / (args.steps * reps)
+    ms_per_step = float(t.item()) / args.steps
     value = world * px_per_frame / (ms_per_step * 1e-3) / 1e6
-    put_per_frame = (pipe.bytes_put - put0) // max(1, args.steps * reps)
+    put_per_frame = (pipe.bytes_put - put0) // max(1, args.steps)
+    if args.dump_outputs and rank == 0:            # the displayed picture of this rank's last timed frame
+        last = pipe.submitted - 1
+        dump_outputs(args.dump_outputs, picture_arrays("picture_", Ss[last % nsets % distinct], pipe.output(last, sets[0].out_name)))
 
     stage_ms = stage_times(torch, lib, sets, nsets)
 
@@ -873,7 +892,7 @@ def run_ours_gop(args):
                 "vs_baseline": None, "dtype": wl["dtype"], "data": "synthetic",
                 "config": {"workload": "%s: %s" % (args.workload, wl["desc"]),
                            "stream": "one dependent stream: frame n on rank n mod %d predicts from the restored pictures of frames n-1 and n-2" % world,
-                           "inner_reps": reps, "timed_region_ms": ms_per_step * args.steps * reps,
+                           "timed_region_ms": ms_per_step * args.steps,
                            "frames_in_flight_per_gpu": n_streams, "band_rows": band_rows, "bands_per_frame": pipe.nb,
                            "cuda_graphs": "one graph launch per frame (bands, waits, puts captured once per frame set; flag values derived on the device from the frame's sequence word)" if graphs else "off",
                            "l2": "%d rotating frame sets per GPU (~%d MB) > 126 MB L2" % (nsets, nsets * ((2 + 2 + fb0.job.run_cdef + fb0.job.run_lr + fb0.job.run_fg) * Ss[0]["pic"].nbytes + Ss[0]["coefs"].nbytes) // 1000000),
@@ -988,6 +1007,8 @@ def run_ours_itx(args):
         ev[i + 1].record()
     sync_all()
     launches = lib.b200_launch_count() - launches0
+    if args.dump_outputs and rank == 0:            # the picture the last timed step wrote into
+        dump_outputs(args.dump_outputs, {"picture": sets[(args.steps - 1) % nsets][2].cpu().numpy()})
     total_ms = ev[0].elapsed_time(ev[-1])
     kern_ms = [ev[i].elapsed_time(ev[i + 1]) for i in range(args.steps)]
     t = torch.tensor([total_ms], device="cuda")
@@ -1063,6 +1084,22 @@ def emit(line):
     out.flush()
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """arrays (name -> numpy) as dirname/<name>.npy in float32; above DUMP_BYTES in all, each array is cut down to the
+    same fixed seeded sample of its flattened elements (sorted indices)"""
+    os.makedirs(dirname, exist_ok=True)
+    total = sum(a.size for a in arrays.values()) * 4
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if total > DUMP_BYTES:
+            keep = max(1, a.size * DUMP_BYTES // total)
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 def main():
     # stdout carries the JSON line and nothing else: libraries that print to fd 1 (e.g. NCCL's version banner) go to stderr
     global _JSON_OUT
@@ -1073,6 +1110,8 @@ def main():
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step as DIR/<name>.npy (float32, at most 64 MB)")
     ap.add_argument("--workload", default="4k8_inter", choices=["4k8_inter", "4k8_mixed", "4k10_full", "8k10_full", "1080p8_intra", "itx8x8"] + sorted(STREAM_WORKLOADS))
     args = ap.parse_args()
     if args.workload in STREAM_WORKLOADS:

@@ -1,8 +1,8 @@
 """Host glue for decoding AV1 elementary streams with the B200 back end behind a real dav1d front end.
 
-`integration/_ref/libdav1d_b200.so` is the unmodified dav1d library whose `f->bd_fn` hooks are the record emitters of
-integration/dav1d/ (built by integration/dav1d/Makefile where the reference sources exist; it travels prebuilt to the
-GPU box). This module binds its stream driver (dav1d's public API: dav1d_open / dav1d_send_data / dav1d_get_picture)
+`oracle/_ref/libdav1d_b200.so` is the unmodified dav1d library whose `f->bd_fn` hooks are the record emitters of
+integration/dav1d/ (built by integration/dav1d/Makefile where the reference sources exist; like the rest of oracle/_ref/
+it is shipped prebuilt to machines without them). This module binds its stream driver (dav1d's public API: dav1d_open / dav1d_send_data / dav1d_get_picture)
 and points the hooks at dav1d_b200/libb200av1.so. No CPU fallback: without the CUDA library the decode fails."""
 import ctypes as C
 import os
@@ -10,8 +10,8 @@ import os
 import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-HOOKED_SO = os.path.join(ROOT, "integration", "_ref", "libdav1d_b200.so")
-LEVEL1_SO = os.path.join(ROOT, "integration", "_ref", "libdav1d_b200_l1.so")
+HOOKED_SO = os.path.join(ROOT, "oracle", "_ref", "libdav1d_b200.so")
+LEVEL1_SO = os.path.join(ROOT, "oracle", "_ref", "libdav1d_b200_l1.so")
 FAMILIES = {"itx": 1, "mc": 2, "ipred": 4, "loopfilter": 8, "cdef": 16, "looprestoration": 32, "filmgrain": 64}
 
 
@@ -23,7 +23,7 @@ class HookStats(C.Structure):
 
 
 def build_hooked(verbose=False):
-    """(Re)build integration/_ref/libdav1d_b200.so (+ the Level-1 variant) where the reference sources exist; a no-op on the GPU box."""
+    """(Re)build oracle/_ref/libdav1d_b200.so (+ the Level-1 variant) where the reference sources exist; a no-op elsewhere."""
     import subprocess
     r = subprocess.run(["make", "-j8", "-C", os.path.join(ROOT, "integration", "dav1d"), "all"], capture_output=True, text=True)
     if r.returncode:
@@ -73,10 +73,7 @@ class HookedDecoder:
 
     def __init__(self, backend=None, serialize=False):
         if not os.path.exists(HOOKED_SO):
-            if os.path.isdir("/root/reference/src"):
-                build_hooked()
-            else:
-                raise RuntimeError("integration/_ref/libdav1d_b200.so missing (it is built where the reference sources exist)")
+            raise RuntimeError("oracle/_ref/libdav1d_b200.so missing (build() makes it where the reference sources exist)")
         if backend is None:
             from . import _lib
             _lib.get_lib()                       # builds / loads the CUDA library or raises
@@ -113,10 +110,7 @@ class Level1Decoder:
 
     def __init__(self, backend=None, families=None):
         if not os.path.exists(LEVEL1_SO):
-            if os.path.isdir("/root/reference/src"):
-                build_hooked()
-            else:
-                raise RuntimeError("integration/_ref/libdav1d_b200_l1.so missing (it is built where the reference sources exist)")
+            raise RuntimeError("oracle/_ref/libdav1d_b200_l1.so missing (build() makes it where the reference sources exist)")
         if backend is None:
             from . import _lib
             backend = _lib.get_lib().path

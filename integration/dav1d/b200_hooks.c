@@ -49,6 +49,8 @@ static HookFrame g_frames[64];
 static B200HookStats g_stats;
 static uint64_t g_clock;            /* LRU stamps of the frame-context and picture tables */
 
+API void b200hook_release(void);
+
 API int b200hook_set_backend(const char *path)
 {
     /* build the table locally, publish it with one release store: a thread that sees g_be_ok set sees every pointer.
@@ -78,6 +80,8 @@ API int b200hook_set_backend(const char *path)
         dlclose(h);
         return -1;
     }
+    /* the frame slots' buffers and streams belong to the back end that allocated them: free them through it first */
+    if (__atomic_load_n(&g_be_ok, __ATOMIC_ACQUIRE)) b200hook_release();
     pthread_mutex_lock(&g_lock);
     g_be = be;
     __atomic_store_n(&g_be_ok, 1, __ATOMIC_RELEASE);

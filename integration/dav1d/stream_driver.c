@@ -4,7 +4,7 @@
  * Decodes an AV1 elementary stream (a list of temporal units) through dav1d's PUBLIC API only
  * (dav1d_open / dav1d_send_data / dav1d_get_picture, reference include/dav1d/dav1d.h, src/lib.c)
  * and packs every output picture tightly into one buffer. It knows nothing about either back end: it is linked
- * into integration/_ref/libdav1d_b200.so (dav1d's front end with the B200 back end behind f->bd_fn) and — by
+ * into oracle/_ref/libdav1d_b200.so (dav1d's front end with the B200 back end behind f->bd_fn) and — by
  * oracle/Makefile — into oracle/_ref/libdav1d_ref.so (the stock CPU decoder = the checker), so a test can compare
  * the two byte for byte.
  */

@@ -1,7 +1,7 @@
 """Test-side access to the three checkers and the checkasm-style input generators.
 
   ref()     oracle/_ref/libdav1d_ref.so — the UNMODIFIED dav1d C path (+ oracle/refdriver);
-            built here by oracle/Makefile, shipped prebuilt to the GPU box (no /root/reference there)
+            built by build() (oracle/Makefile) where the reference sources exist, shipped prebuilt elsewhere
   oracle()  oracle/liboracle.so — this repo's plain-C restatement (always buildable: gcc only)
   emu_lib() tests/emu: the CUDA sources compiled for the host fiber emulator (debug harness)
 """
@@ -26,14 +26,12 @@ def _make(target):
 
 
 def have_ref():
-    if not os.path.exists(REF_SO) and os.path.isdir("/root/reference/src"):
-        _make("ref")
     return os.path.exists(REF_SO)
 
 
 def ref():
     if "ref" not in _cache:
-        assert have_ref(), "oracle/_ref/libdav1d_ref.so missing (build it where /root/reference exists)"
+        assert have_ref(), "oracle/_ref/libdav1d_ref.so missing (build() makes it where the reference sources exist)"
         lib = C.CDLL(REF_SO)
         lib.refdrv_scan.restype = C.POINTER(C.c_uint16)
         lib.refdrv_itx_add_batch.restype = C.c_double

@@ -1,5 +1,5 @@
 """Real-stream drop-in test: the same AV1 elementary stream decoded (a) by the stock reference (oracle/_ref, dav1d's own
-CPU back end) and (b) by integration/_ref/libdav1d_b200.so = the same dav1d front end with the f->bd_fn hooks emitting
+CPU back end) and (b) by oracle/_ref/libdav1d_b200.so = the same dav1d front end with the f->bd_fn hooks emitting
 B200 records and libb200av1 reconstructing + filtering every frame. Output pictures must be byte-identical.
 Streams: dav1d_b200/obu.py (valid headers, random tile payloads: every intra tool, per-block delta q / lf, CDEF, LR).
 CPU tests bind the hooks to the host emulator build of the CUDA sources; GPU tests bind the real library."""
@@ -12,8 +12,8 @@ import pytest
 import refs
 from dav1d_b200 import obu, stream
 
-pytestmark = pytest.mark.skipif(not (os.path.exists(stream.HOOKED_SO) or os.path.isdir("/root/reference/src")),
-                                reason="integration/_ref/libdav1d_b200.so not built")
+pytestmark = pytest.mark.skipif(not (os.path.exists(stream.HOOKED_SO) and refs.have_ref()),
+                                reason="oracle/_ref/libdav1d_b200.so not built")
 
 
 def _ref_decode(tus, **kw):
@@ -51,8 +51,6 @@ def emu_decoder():
     import importlib.util
     spec = importlib.util.spec_from_file_location("build_emu", os.path.join(refs.ROOT, "tests", "emu", "build_emu.py"))
     m = importlib.util.module_from_spec(spec); spec.loader.exec_module(m)
-    if os.path.isdir("/root/reference/src"):
-        stream.build_hooked()
     d = stream.HookedDecoder(backend=m.build(), serialize=True)
     yield d
     d.release()
@@ -358,8 +356,6 @@ def test_stream_without_backend_fails_loudly():
     """no CPU fallback: with no back end bound the hooked decoder reports an error instead of decoding (own process:
     the binding is process-wide state of the library)"""
     import subprocess, sys
-    if os.path.isdir("/root/reference/src"):
-        stream.build_hooked()
     code = ("import ctypes as C, os, sys; sys.path.insert(0, %r); os.environ.pop('B200AV1_LIB', None)\n"
             "from dav1d_b200 import obu, stream\n"
             "dll = C.CDLL(stream.HOOKED_SO)\n"
@@ -487,8 +483,6 @@ def test_hook_wavefront_sort_is_a_valid_order():
     """b200hook_wave_sort (integration/dav1d/b200_hooks.c): the order it produces must keep every intra record behind the
     records whose pixels its edge array reads (the kernel's ticket order requirement), for records in decode order"""
     from dav1d_b200 import synth, levels as L
-    if os.path.isdir("/root/reference/src"):
-        stream.build_hooked()
     dll = C.CDLL(stream.HOOKED_SO)
     S = synth.make_intra_frame(np.random.default_rng(11), 8, 328, 200)
     tx = S["intra_tx_decode_order"]
@@ -530,8 +524,6 @@ def test_cli_md5_y4m_and_obu_file_roundtrip(tmp_path, capsys):
     spec = importlib.util.spec_from_file_location("build_emu", os.path.join(refs.ROOT, "tests", "emu", "build_emu.py"))
     m = importlib.util.module_from_spec(spec); spec.loader.exec_module(m)
     emu = m.build()
-    if os.path.isdir("/root/reference/src"):
-        stream.build_hooked()
     obu_file, y4m = str(tmp_path / "s.obu"), str(tmp_path / "o.y4m")
     assert cli.main(["--synth", "inter:208x144:10:3:grain,mm", "-w", obu_file]) == 0
     tus = cli.split_temporal_units(open(obu_file, "rb").read())
@@ -609,7 +601,7 @@ def test_golden_streams_hooked_emu_md5(emu_decoder):
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["key_8bit_tiles", "inter_10bit_all_tools"])
 def test_golden_streams_hooked_gpu_md5(gpu_decoder, name):
-    """needs neither /root/reference nor oracle/: the digest of the reference's output is committed"""
+    """compares with no reference decode: the digest of the reference's output is committed"""
     tus, want = _golden()[name]
     assert _md5(gpu_decoder.decode(tus, apply_grain=1)) == (want["md5"], want["frames"])
     gpu_decoder.stats(reset=True)
@@ -638,8 +630,6 @@ def test_level1_tables_inside_dav1d_emu():
     spec = importlib.util.spec_from_file_location("build_emu", os.path.join(refs.ROOT, "tests", "emu", "build_emu.py"))
     m = importlib.util.module_from_spec(spec); spec.loader.exec_module(m)
     emu_path = m.build()
-    if os.path.isdir("/root/reference/src"):
-        stream.build_hooked()
     emu = refs.emu_lib()
     _level1_case(stream.Level1Decoder(backend=emu_path), lambda: int(emu.b200_launch_count()))
 

@@ -2,14 +2,14 @@
 """Fuzz the hooked decoder against stock dav1d on the CPU: randomly parameterised synthetic streams (every header option of
 dav1d_b200/obu.py drawn at random: bit depth, layout, superblock size, tiles, film grain, screen content + intra block copy,
 motion modes, global motion, segmentation, hidden / intra-only frames, changing frame sizes, super-resolution), decoded with
-random thread counts / frames in flight through integration/_ref/libdav1d_b200.so bound to the host-emulator build of the CUDA
+random thread counts / frames in flight through oracle/_ref/libdav1d_b200.so bound to the host-emulator build of the CUDA
 sources, and through oracle/_ref (stock dav1d); every output picture must be byte-identical. Streams the stock decoder rejects
 (random payloads are not always legal, e.g. 4:2:2 or intra block copy) are skipped. Every other stream goes through the stream
 generator first (tests/streamgen.py: symbols chosen and range-encoded by the reference decoder itself), with a random policy for
 skipped blocks / sparse coefficients / intra share — and, for 4:2:2, frames of any size, since the generator avoids the
 partitions that are illegal there.
 usage: tools/fuzz_streams.py [n_streams] [first_seed] [big | level1]
-   big: frames up to 1000x560 instead of 420x290;  level1: small frames through integration/_ref/libdav1d_b200_l1.so instead — dav1d's
+   big: frames up to 1000x560 instead of 420x290;  level1: small frames through oracle/_ref/libdav1d_b200_l1.so instead — dav1d's
    own reconstruction code on the B200 function tables (every Dav1dDSPContext slot incl. mc_scaled / resize / emu_edge / warp / blend),
    one emulated kernel launch per DSP call"""
 import importlib.util
