@@ -171,7 +171,7 @@ class FrameBand(C.Structure):
     """struct B200FrameBand"""
     _fields_ = [("y0", C.c_int32), ("y1", C.c_int32), ("last", C.c_int32), ("pad", C.c_int32)] + \
                [(n, C.c_int32 * 2) for n in ("pred", "warp", "comp", "comp2", "blend", "blend2", "scaled", "cfused", "cfused2", "expand")] + \
-               [("itx", (C.c_int32 * 2) * 19)]
+               [("itx", (C.c_int32 * 2) * 19), ("intra", C.c_int32 * 2), ("edge_top", C.c_void_p), ("edge_bottom", C.c_void_p)]
 
 
 class PutRange(C.Structure):

@@ -123,8 +123,17 @@ int b200_frame_run_band_phase(const B200FrameJob *j, const B200FrameBand *b, int
         return -2;
     }
     const bool first = b->y0 == 0;
-    // intra records form a dependency graph over the whole frame: they run with a band only when that band IS the frame
-    if (j->n_intra > 0 && !(first && b->last)) { b200_set_error("b200_frame_run_band: intra records are not band-sliced (one band, or b200_frame_run)"); return -2; }
+    // intra records: the band's own range of d_intra, in a topological order of the dependencies inside the band (those on
+    // the bands above are met); a record on the band's first row reads its top edge from the rows the band above saved
+    if (j->n_intra > 0) {
+        if (b->intra[0] < 0 || b->intra[1] < 0 || b->intra[1] > j->n_intra - b->intra[0]) {
+            b200_set_error("b200_frame_run_band: intra records [%d, +%d) outside [0, %d)", b->intra[0], b->intra[1], j->n_intra);
+            return -2;
+        }
+        if (j->intra.sb && !(first && b->last)) { b200_set_error("b200_frame_run_band: the superblock-granular intra schedule is not band-sliced (one band, or b200_frame_run)"); return -2; }
+        if (!first && b->intra[1] > 0 && !b->edge_top) { b200_set_error("b200_frame_run_band: band [%d, %d) has intra records but no edge_top", b->y0, b->y1); return -2; }
+        if (!b->last && !b->edge_bottom) { b200_set_error("b200_frame_run_band: band [%d, %d) of a job with intra records has no edge_bottom", b->y0, b->y1); return -2; }
+    }
     if (j->run_resize) { b200_set_error("b200_frame_run_band: the super-resolution stage is not band-sliced (b200_frame_run)"); return -2; }
     // (the grain LUTs belong to the post phase: its stream forks the preparation beside the first band and joins it before
     // the last band's application)
@@ -159,7 +168,11 @@ int b200_frame_run_band_phase(const B200FrameJob *j, const B200FrameBand *b, int
         itx_n[t] = j->d_itx[t] ? b->itx[t][1] : 0;
     }
     if ((r = b200_itx_add_frame(bd, itx_p, itx_n, j->d_coef, j->mc.dst, j->itx_stride, j->zero_coefs, stream))) return r;
-    if (j->n_intra > 0 && (r = b200_intra_frame(bd, &j->intra, j->d_intra, j->n_intra, stream))) return r;
+    if (j->n_intra > 0) {
+        if ((r = b200::intra_band(bd, &j->intra, j->d_intra + b->intra[0], b->intra[1], first, (cudaStream_t)stream))) return r;
+        // the band's last rows, before its post filters change them: the top edge of the band below (launch + ticket reset)
+        if (!b->last && (r = b200::intra_edge_backup(bd, &j->intra, b->y1, b->edge_bottom, (cudaStream_t)stream))) return r;
+    }
     }
     if (!do_post) return 0;
     // sweeps: what this band's reconstruction makes final. Deblock: the band's own rows (a row-edge filter at y1 will still

@@ -40,6 +40,10 @@ std::mutex &host_lock();
 
 // row-range forms of the frame-wide sweeps (a band of a frame job, frame.cu; the b200_*_frame entry points pass the whole range)
 int lf_frame_rows(int bdmax, const B200LfFrame *f, int ya4, int yb4, cudaStream_t stream);
+// band-sliced intra stage (intra.cu): the records of one band (first: the done map is set up from done_init / zeroed
+// first, also when the band has no records), and the edge rows the band below reads (intra.scratch header -> band y1)
+int intra_band(int bdmax, const B200IntraFrame *f, const B200IntraTx *d_tx, int n, bool first, cudaStream_t stream);
+int intra_edge_backup(int bdmax, const B200IntraFrame *f, int y1, void *edge, cudaStream_t stream);
 int cdef_frame_rows(int bdmax, const B200CdefFrame *f, int t0, int t1, cudaStream_t stream);
 int lr_frame_rows(int bdmax, const B200LrFrame *f, int r0, int r1, cudaStream_t stream);
 

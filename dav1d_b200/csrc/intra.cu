@@ -27,7 +27,17 @@
 
 namespace b200 {
 
-// scratch layout: [ticket counter: 256 B][done maps of the three planes, one byte per 4x4 cell]
+// scratch layout: [header: 256 B][done maps of the three planes, one byte per 4x4 cell]
+// The header holds the ticket counter and the band the next launch reconstructs. A band-sliced job (b200_frame_run_band)
+// launches the kernel once per band; the edge-backup kernel of band k-1 resets the ticket and points `edge` at the row
+// of each plane just above band k, saved before that row was deblocked (dav1d's f->ipred_edge, reference
+// src/recon_tmpl.c:2111-2135). Records on the band's first row take their top edge from there. All zero (the state
+// b200_intra_frames starts from): no band, every edge comes from the picture.
+struct IntraHdr {
+    int ticket;
+    int band_y;                 // luma row where the band starts (its first chroma row: band_y >> ss_ver)
+    const void *edge;           // NULL, or the Y, U and V rows above band_y, each `stride[p]` samples long, back to back
+};
 struct IntraScratch {
     size_t done_off[3], total;
 };
@@ -70,6 +80,21 @@ struct IntraBatch { IntraParams p[kIntraMaxBatch]; };
 static_assert(sizeof(IntraBatch) <= 4080, "kernel parameter space (4 KB with the trailing int)");
 
 B200_DEV int ld_cell(const uint8_t *p) { return *(const volatile uint8_t *)p; }
+// the row above a block: the picture's, or the saved edge row when the block starts the band (its row above belongs to
+// the previous band, whose post filters may already be rewriting it). The header is read only on the first row of a
+// 64-luma-row superblock row (bands start there): nothing stays live across the loop.
+template <class pixel, class Frame>
+B200_DEV const pixel *top_row(const Frame &f, const uint8_t *scratch, const pixel *dst, int pl, int x4, int y4)
+{
+    const int ssv = pl ? f.ss_ver : 0;
+    if (!((y4 * 4) & (63 >> ssv))) {
+        const IntraHdr *const hdr = (const IntraHdr *)scratch;
+        const void *const edge = hdr->edge;
+        if (edge && (y4 * 4) << ssv == hdr->band_y)
+            return (const pixel *)edge + (pl ? f.stride[0] + (pl - 1) * f.stride[1] : 0) + x4 * 4;
+    }
+    return dst - f.stride[pl];
+}
 // a dependency that never arrives (records not in a topological order) must not hang the GPU: fail the launch
 B200_DEV void intra_stuck() {
 #ifndef B200_EMU
@@ -256,7 +281,7 @@ __global__ void __launch_bounds__(kIpT, B200_INTRA_MINB) intra_frame_kernel(cons
         }
         // ---- edge gather (every part is filled; the predictors read only what the reference fills)
         {
-            const pixel *const top = dst - st;
+            const pixel *const top = top_row(f, P.scratch, dst, pl, x, y);
             const int half = (1 << bitdepth) >> 1;
             const int lpx = imin(h, (ye - y) << 2), lpx2 = imin(h, (ye - y - th) << 2);
             const int tpx = imin(w, (xe - x) << 2), tpx2 = imin(w, (xe - x - tw) << 2);
@@ -527,7 +552,7 @@ __global__ void __launch_bounds__(kIwWarps * 32) intra_warp_kernel(const __grid_
         }
         // ---- edge gather (every part is filled; the predictors read only what the reference fills)
         if (!is_resid && !is_pal && !is_ibc) {
-            const pixel *const top = dst - st;
+            const pixel *const top = top_row(f, P.scratch, dst, pl, x, y);
             const int half = (1 << bitdepth) >> 1;
             const int lpx = imin(h, (ye - y) << 2), lpx2 = imin(h, (ye - y - th) << 2);
             const int tpx = imin(w, (xe - x) << 2), tpx2 = imin(w, (xe - x - tw) << 2);
@@ -854,9 +879,74 @@ __global__ void __launch_bounds__(kIpT, B200_INTRA_SB_MINB) intra_sb_kernel(cons
     }
 }
 
+// ---- band-sliced jobs: the rows band k+1 reads from above ---------------------------------------------------------
+// Run at the end of band k's reconstruction, before its post filters: copies the last row of each plane of the band
+// (luma y1 - 1, chroma (y1 >> ss_ver) - 1, `stride` samples each) into `edge`, then sets the header up for band k+1's
+// launch (ticket 0, band row y1, edge). One CTA per plane.
+struct EdgeBackupArgs {
+    const unsigned char *src[3];
+    uint32_t bytes[3], dst_off[3];
+    unsigned char *edge;
+    IntraHdr *hdr;
+    int band_y;
+};
+constexpr int kEdgeThreads = 256;
+__global__ void __launch_bounds__(kEdgeThreads) intra_edge_backup_kernel(const __grid_constant__ EdgeBackupArgs a)
+{
+    const int p = blockIdx.x;
+    const unsigned char *const src = a.src[p];
+    unsigned char *const dst = a.edge + a.dst_off[p];
+    const uint32_t n = a.bytes[p];
+    if (!(((uintptr_t)src | (uintptr_t)dst | n) & 3)) {
+        for (uint32_t i = threadIdx.x; i < n >> 2; i += kEdgeThreads) ((uint32_t *)dst)[i] = ((const uint32_t *)src)[i];
+    } else {
+        for (uint32_t i = threadIdx.x; i < n; i += kEdgeThreads) dst[i] = src[i];
+    }
+    if (p == 0 && threadIdx.x == 0) { a.hdr->ticket = 0; a.hdr->band_y = a.band_y; a.hdr->edge = a.edge; }
+}
+
+int intra_edge_backup(int bdmax, const B200IntraFrame *f, int y1, void *edge, cudaStream_t stream)
+{
+    const size_t px = bdmax > 255 ? 2 : 1;
+    EdgeBackupArgs a;
+    memset(&a, 0, sizeof(a));
+    uint32_t o = 0;
+    for (int p = 0; p < 3; p++) {
+        const int row = (p ? y1 >> f->ss_ver : y1) - 1;
+        a.src[p] = (const unsigned char *)f->pic + (f->plane_off[p] + (size_t)row * f->stride[p]) * px;
+        a.bytes[p] = (uint32_t)(f->stride[p] * px);
+        a.dst_off[p] = o;
+        o += a.bytes[p];
+    }
+    a.edge = (unsigned char *)edge;
+    a.hdr = (IntraHdr *)f->scratch;
+    a.band_y = y1;
+    B200_LAUNCH(intra_edge_backup_kernel, dim3(3), dim3(kEdgeThreads), 0, stream, a);
+    b200_count_launch();
+    B200_CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
 }  // namespace b200
 
 using namespace b200;
+
+static int intra_frames_impl(int bdmax, const B200IntraFrame *frames, const B200IntraTx *const *d_tx, const int32_t *n_tx,
+                             int n_frames, bool init, void *stream);
+
+namespace b200 {
+int intra_band(int bdmax, const B200IntraFrame *f, const B200IntraTx *d_tx, int n, bool first, cudaStream_t stream)
+{
+    if (n > 0) return intra_frames_impl(bdmax, f, &d_tx, &n, 1, first, stream);
+    if (!first) return 0;
+    // a first band without intra records still sets the done map up for the bands below it
+    if (!f->scratch) { b200_set_error("b200_frame_run_band: no intra scratch"); return -2; }
+    const IntraScratch L = intra_scratch_layout(f);
+    if (f->done_init) B200_CUDA_OK(cudaMemcpyAsync(f->scratch, f->done_init, L.total, cudaMemcpyDeviceToDevice, stream));
+    else B200_CUDA_OK(cudaMemsetAsync(f->scratch, 0, L.total, stream));
+    return 0;
+}
+}  // namespace b200
 
 extern "C" {
 
@@ -874,6 +964,16 @@ static size_t intra_canvas_bytes(const B200IntraFrame *f, size_t px)
 
 int b200_intra_frames(int bdmax, const B200IntraFrame *frames, const B200IntraTx *const *d_tx, const int32_t *n_tx,
                       int n_frames, void *stream)
+{
+    return intra_frames_impl(bdmax, frames, d_tx, n_tx, n_frames, true, stream);
+}
+
+}  // extern "C"
+
+// init: set the scratch up (done map from done_init or zeroed, header zeroed) before the launch; false: a later band of a
+// band-sliced job, whose done map holds the bands above and whose header the edge-backup kernel has set
+static int intra_frames_impl(int bdmax, const B200IntraFrame *frames, const B200IntraTx *const *d_tx, const int32_t *n_tx,
+                             int n_frames, bool init, void *stream)
 {
     if (bdmax != 255 && bdmax != 1023 && bdmax != 4095) { b200_set_error("b200_intra_frames: bad bitdepth_max"); return -2; }
     const size_t px = bdmax > 255 ? 2 : 1;
@@ -899,7 +999,9 @@ int b200_intra_frames(int bdmax, const B200IntraFrame *frames, const B200IntraTx
             uint8_t *base_p = (uint8_t *)f->scratch;
             P.scratch = base_p;
             for (int p = 0; p < 3; p++) P.done_off[p] = (uint32_t)L.done_off[p];
-            if (!mode && f->done_init)
+            if (!init)
+                ;
+            else if (!mode && f->done_init)
                 B200_CUDA_OK(cudaMemcpyAsync(base_p, f->done_init, L.total, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
             else
                 B200_CUDA_OK(cudaMemsetAsync(base_p, 0, mode ? 256 + (size_t)f->sb_w * f->sb_h : L.total, (cudaStream_t)stream));
@@ -944,6 +1046,8 @@ int b200_intra_frames(int bdmax, const B200IntraFrame *frames, const B200IntraTx
     }
     return 0;
 }
+
+extern "C" {
 
 int b200_intra_frame(int bdmax, const B200IntraFrame *f, const B200IntraTx *d_tx, int n, void *stream)
 {

@@ -78,12 +78,18 @@ def band_plan(S, band_rows, compact=False, fused=False):
     order is kept inside a band), bands = list of dicts {y0, y1, last, <record list>: (first, count)} and need[k][ref] =
     (luma rows, chroma rows) of reference `ref` that band k's predictions read — the `lowest_pixel` of dav1d's
     check_tile (reference src/thread_task.c:415, src/decode.c lowest_pixel bookkeeping); expand = the compact coefficient
-    stream and its band-sorted B200CoefBlock records when `compact`."""
+    stream and its band-sorted B200CoefBlock records when `compact`.
+    Intra-machine records (S["intra_tx"]) are sorted by band too, keeping their wavefront order inside a band. A band may
+    only depend on itself and the bands above it: ValueError when a record's bottom-left edge or an intra block copy's
+    source reaches below its band (band edges must fall on superblock rows), and when the frame has predictions from
+    scaled references (not band-sliced)."""
     assert band_rows % 64 == 0 and band_rows > 0
     H, off, stride = S["H"], S["off"], S["stride"]
     ssv = [0, S["ss_ver"], S["ss_ver"]]
     nb = -(-H // band_rows)
     S2 = dict(S)
+    if nb > 1 and S.get("scaled") is not None and len(S["scaled"]):
+        raise ValueError("band_plan: predictions from scaled references are not band-sliced (one band)")
 
     def luma_y(dst_off, plane):
         pl = np.asarray(plane).astype(np.int64)
@@ -98,7 +104,7 @@ def band_plan(S, band_rows, compact=False, fused=False):
         first = np.concatenate([[0], np.cumsum(cnt)[:-1]])
         return arr[order], first, cnt, band[order]
 
-    ranges = {}
+    ranges, band_of = {}, {}
     # compound records first: they tell where the int16 predictions (op 1, addressed in `tmp`) belong
     tmp_y = {}
     for name in ("comp", "comp2"):
@@ -117,7 +123,7 @@ def band_plan(S, band_rows, compact=False, fused=False):
             if name != "warp":
                 for t, yy in zip(a["tmp_off"].tolist(), y.tolist()):
                     lap_y[t] = yy
-            S2[name], f, c, _ = sort_by_band(a, y)
+            S2[name], f, c, band_of[name] = sort_by_band(a, y)
             ranges[name] = (f, c)
     pname = "pred_single" if (fused and "cfused" in S) else "pred"
     a = S[pname]
@@ -134,8 +140,14 @@ def band_plan(S, band_rows, compact=False, fused=False):
     for name in ("cfused", "cfused2"):
         if fused and name in S:
             a = S[name]
-            S2[name], f, c, _ = sort_by_band(a, luma_y(a["dst_off"], a["plane"]) if len(a) else np.zeros(0, np.int64))
+            S2[name], f, c, band_of[name] = sort_by_band(a, luma_y(a["dst_off"], a["plane"]) if len(a) else np.zeros(0, np.int64))
             ranges[name] = (f, c)
+    iband = None
+    it = S.get("intra_tx")
+    if it is not None and len(it):
+        S2["intra_tx"], f, c, iband = sort_by_band(it, it["y4"].astype(np.int64) * 4 << np.asarray(ssv, np.int64)[it["plane"]])
+        ranges["intra"] = (f, c)
+        _check_intra_bands(S2["intra_tx"], iband, band_rows, nb, S)
     S2["itx"] = {}
     itx_ranges = {}
     for tx in range(19):
@@ -149,9 +161,11 @@ def band_plan(S, band_rows, compact=False, fused=False):
         # compact_coefs emits its records size class after size class, each in the (band-sorted) order of S2["itx"][tx]
         per_tx = [np.repeat(np.arange(nb), itx_ranges[tx][1]) for tx in range(19) if len(S2["itx"][tx])]       # empty: every inter block skipped
         eb = np.concatenate(per_tx) if per_tx else np.zeros(0, np.int64)
-        # ... followed by the intra records' blocks (mixed frames: a single band only, see b200_frame_run_band)
-        assert len(eb) == len(ex) or (nb == 1 and len(eb) < len(ex))
-        eb = np.concatenate([eb, np.zeros(len(ex) - len(eb), np.int64)]).astype(np.int64)
+        # ... followed by the intra records' blocks, size class after size class in the (band-sorted) order of S2["intra_tx"]
+        if iband is not None:
+            t = S2["intra_tx"]
+            eb = np.concatenate([eb] + [iband[(t["tx"] == tx) & (t["eob"] >= 0)] for tx in range(19)]).astype(np.int64)
+        assert len(eb) == len(ex)
         order = np.argsort(eb, kind="stable")
         cnt = np.bincount(eb, minlength=nb)
         expand = (cc, ex[order])
@@ -171,9 +185,52 @@ def band_plan(S, band_rows, compact=False, fused=False):
         low = P["src_y"].astype(np.int64) + P["h"] + 4
         cls = (P["plane"] > 0).astype(np.int64)
         np.maximum.at(need, (pband, P["ref"].astype(np.int64), cls), low)
+    # warps read their reference directly (15 x 15 window: rows src_y - 3 .. src_y + 11); fused compound records carry
+    # both references
+    if "warp" in band_of and len(S2["warp"]):
+        a = S2["warp"]
+        np.maximum.at(need, (band_of["warp"], a["ref"].astype(np.int64), (a["plane"] > 0).astype(np.int64)),
+                      a["src_y"].astype(np.int64) + 12)
+    for name in ("cfused", "cfused2"):
+        if name in band_of and len(S2[name]):
+            a = S2[name]
+            for i in range(2):
+                np.maximum.at(need, (band_of[name], a["ref"][:, i].astype(np.int64), (a["plane"] > 0).astype(np.int64)),
+                              a["src_y"][:, i].astype(np.int64) + a["h"] + 4)
     ph = [H, (H + ssv[1]) >> ssv[1]]
     need[:, :, 0] = np.minimum(need[:, :, 0], ph[0]); need[:, :, 1] = np.minimum(need[:, :, 1], ph[1])
     return S2, bands, need, expand
+
+
+def _check_intra_bands(t, band, band_rows, nb, S):
+    """ValueError when an intra record of a band-sliced frame depends on rows below its band (band = band index per record):
+    the band's launch could never see them (the kernel would trap, or read pixels not yet reconstructed)."""
+    if nb == 1:
+        return
+    from . import levels as L
+    ssv = np.array([0, S["ss_ver"], S["ss_ver"]], np.int64)
+    pl = t["plane"].astype(np.int64)
+    y, th = t["y4"].astype(np.int64), np.asarray(L.TX_H, np.int64)[t["tx"]] // 4
+    ye = t["yend4"].astype(np.int64)
+    # first plane row (in 4-sample units for the edges, samples for the copies) below each record's band; none for the last band
+    end_px = np.where(band < nb - 1, ((band + 1) * band_rows) >> ssv[pl], 1 << 30)
+    flags = t["flags"].astype(np.int64)
+    bl = (flags & 1 != 0) & (flags & 8 != 0) & (y + th < ye)
+    reach = np.minimum(y + 2 * th, ye) * 4
+    bad = bl & (reach > end_px)
+    if bad.any():
+        i = int(np.nonzero(bad)[0][0])
+        raise ValueError("band_plan: intra record %d (plane %d, row %d) reads bottom-left rows down to %d, below its band "
+                         "(band edges must fall on superblock rows)" % (i, pl[i], y[i] * 4, reach[i]))
+    ibc = t["mode"] == 18
+    if ibc.any():
+        ph = np.array([S["h4"], S["h4"] >> S["ss_ver"], S["h4"] >> S["ss_ver"]], np.int64)[pl] * 4
+        sy = t["luma_off"].astype(np.int64) >> 16
+        last = np.minimum(sy + th * 4 - 1 + (t["cfl_h_pad"] != 0), ph - 1)
+        bad = ibc & (last >= end_px)
+        if bad.any():
+            i = int(np.nonzero(bad)[0][0])
+            raise ValueError("band_plan: intra block copy %d (plane %d) copies from row %d, below its band" % (i, pl[i], last[i]))
 
 
 def run_batch(fbs, stream=None):
@@ -229,7 +286,7 @@ class FrameBuffers:
             for k, b in enumerate(plan):
                 fbn = self.bands[k]
                 fbn.y0, fbn.y1, fbn.last = b["y0"], b["y1"], b["last"]
-                for name in ("pred", "warp", "comp", "comp2", "blend", "blend2", "cfused", "cfused2", "expand"):
+                for name in ("pred", "warp", "comp", "comp2", "blend", "blend2", "cfused", "cfused2", "expand", "intra"):
                     if name in b:
                         getattr(fbn, name)[0], getattr(fbn, name)[1] = b[name]
                 for tx in range(19):
@@ -303,8 +360,10 @@ class FrameBuffers:
             it.pic, it.d_coef, it.zero_coefs, it.grid = p0, j.d_coef, 0, intra_grid
             it.ss_hor, it.ss_ver = S["ss_hor"], S["ss_ver"]
             it.mask = mask                            # blend masks of inter-intra (II) records
+            if S.get("intra_pal") is not None:       # colours + index maps of palette (PAL) records
+                it.pal = up("intra_pal", S["intra_pal"]); self.uploads.append(("intra_pal", S["intra_pal"]))
             for p in range(3):
-                it.stride[p] = S["stride"][p]
+                it.stride[p] = S["stride"][p]; it.plane_off[p] = S["off"][p]
                 it.w4[p] = S["w4"] >> ssh[p]; it.h4[p] = S["h4"] >> ssv[p]
             nb = self.lib.b200_intra_scratch_bytes(C.byref(it)) if hasattr(self.lib, "b200_intra_scratch_bytes") else 1 << 22
             it.scratch = zeros("intra_scratch", nb)
@@ -314,8 +373,6 @@ class FrameBuffers:
                 it.sb = up("intra_sb", S["intra_sb"]); it.n_sb = len(S["intra_sb"])
                 it.sb_w, it.sb_h = S["intra_sb_grid"]
                 self.uploads.append(("intra_sb", S["intra_sb"]))
-                for p in range(3):
-                    it.plane_off[p] = S["off"][p]
             else:
                 j.d_intra = up("intra_tx", S["intra_tx"]); j.n_intra = len(S["intra_tx"])
                 self.uploads.append(("intra_tx", S["intra_tx"]))
@@ -323,6 +380,15 @@ class FrameBuffers:
                     it.done_init = up("done_init", S["done_init"])
                     self.uploads.append(("done_init", S["done_init"]))
             n_intra = 1
+            if self.bands is not None and len(self.bands) > 1:
+                if (S["intra_tx"]["mode"] == 18).any() and (run_lf or run_cdef or run_lr):
+                    raise ValueError("intra block copy reads the unfiltered picture above its band: its frames run with "
+                                     "deblocking, CDEF and loop restoration off")
+                # the rows each band saves for the band below (B200FrameBand.edge_top / edge_bottom): Y, U, V rows back to back
+                eb = sum(S["stride"]) * px
+                base = zeros("band_edges", eb * (len(self.bands) - 1))
+                for k in range(len(self.bands) - 1):
+                    self.bands[k].edge_bottom = self.bands[k + 1].edge_top = base + k * eb
         # post filters
         j.run_lf, j.run_cdef, j.run_lr = int(run_lf), int(run_cdef), int(run_lr)
         d_masks = up("masks", S["masks"]); self.uploads.append(("masks", S["masks"]))

@@ -546,7 +546,7 @@ typedef struct B200IntraFrame {
     int32_t zero_coefs;
     int32_t grid;                  /* CTAs to launch; 0 = default */
     void *scratch;                 /* device, >= b200_intra_scratch_bytes(frame) */
-    uint32_t plane_off[3];         /* superblock mode: sample offset of each plane in pic */
+    uint32_t plane_off[3];         /* superblock mode and band-sliced jobs: sample offset of each plane in pic */
     int32_t n_sb, sb_w, sb_h;      /* superblock mode: number of B200IntraSb, superblock grid */
     const B200IntraSb *sb;         /* device; NULL = per-transform-block dataflow */
     const uint8_t *mask;           /* device or NULL: blend masks of B200_INTRA_MODE_II records (per-transform-block mode only) */
@@ -654,7 +654,22 @@ B200_API int b200_struct_size(int which);
  *       CDEF tile rows (32 luma rows) below y1 - 32, loop-restoration tile rows whose stripe ends at or above y1 - 8,
  *     and, for the last band, everything down to the bottom edge + film grain.
  * After band k the restored picture is final down to b200_band_progress(): the rows a dependent frame may predict from.
- * Bands must be run in order, top to bottom, on one stream; the result is bit-identical to b200_frame_run. */
+ * Bands must be run in order, top to bottom, on one stream; the result is bit-identical to b200_frame_run.
+ * Intra records (d_intra, per-transform-block schedule) are band-sliced too: band k runs records [intra[0], +intra[1]),
+ * a topological order of their dependencies inside the band, after its inter stages. A record may depend on anything in
+ * its own band or above, never below: bands fall on superblock rows, and no bottom-left edge or intra-block-copy source
+ * reaches below the band's last row (with 128x128 superblocks a band edge inside a superblock can break this; such plans
+ * are the caller's to reject). The done map is set up once, by the top band (from intra.done_init, or zeroed). Since the
+ * post filters of band k may rewrite its last rows while band k+1 is reconstructed, the reconstruction of band k ends by
+ * saving the last row of each plane (luma y1 - 1, chroma (y1 >> ss_ver) - 1; dav1d's f->ipred_edge, reference
+ * src/recon_tmpl.c:2111-2135) into edge_bottom, and band k+1's records on its first row read their top edge (top-left,
+ * top-right included) from there: its edge_top is band k's edge_bottom. An edge buffer holds the Y, U and V rows back to
+ * back, intra.stride[p] samples each; the rows are read at intra.plane_off[p] of intra.pic, which band-sliced jobs with
+ * intra records must fill. Both are needed only when the job has intra records: edge_top when y0 > 0 and the band has
+ * records, edge_bottom unless the band is the bottom one. Intra block copy reads the picture above directly, which is
+ * only valid because such frames run with deblocking, CDEF and loop restoration off. The superblock-granular schedule
+ * (intra.sb) runs as a single band only. b200_frame_run_band_phase returns -2, before enqueueing anything, on a band
+ * that breaks these rules where it can see it without reading device memory. */
 typedef struct B200FrameBand {
     int32_t y0, y1;                 /* luma rows reconstructed by this band */
     int32_t last;                   /* 1: bottom band (y1 = picture height; sweeps run to the bottom edge) */
@@ -662,6 +677,9 @@ typedef struct B200FrameBand {
     /* [first, count) of the job's record arrays that belong to this band */
     int32_t pred[2], warp[2], comp[2], comp2[2], blend[2], blend2[2], scaled[2], cfused[2], cfused2[2], expand[2];
     int32_t itx[B200_N_RECT_TX_SIZES][2];
+    int32_t intra[2];               /* [first, count) of d_intra (see below) */
+    void *edge_top;                 /* device: the rows above y0 that the band above saved (NULL for the top band) */
+    void *edge_bottom;              /* device: where this band saves its last rows (NULL for the bottom band) */
 } B200FrameBand;
 B200_API int b200_frame_run_band(const B200FrameJob *job, const B200FrameBand *band, void *stream);
 /* The two halves of a band for callers that pipeline them on two streams: B200_BAND_RECON = coefficient expansion,

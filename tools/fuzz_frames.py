@@ -2,7 +2,7 @@
 """Fuzz the frame job against the oracle on the CPU: random synthetic frames (dav1d_b200/synth.py: bit depth, chroma layout, frame
 size, compound / skip / intra / OBMC / warp / inter-intra rates, film grain; intra-only frames with intra block copy) through the
 host-emulator build of the CUDA sources — whole-frame job, compact coefficient upload, fused compound prediction, band-sliced
-execution with random band heights — compared with oracle/*.c stage by stage (tests/test_frame.py::check_frame).
+execution with random band heights (intra-only frames too, filters off) — compared with oracle/*.c stage by stage (tests/test_frame.py::check_frame).
 usage: tools/fuzz_frames.py [n_frames] [first_seed]"""
 import os
 import sys
@@ -34,6 +34,12 @@ def main():
                 got = TI.run_lib(lib, frame.NumpyAlloc(), S, order=str(rng.choice(["intra_tx", "intra_tx_decode_order"])), compact=bool(rng.integers(0, 2)))
                 ok, where = TI.planes_equal(S, exp, got)
                 assert ok, where
+                # band by band (intra block copy reads the unfiltered picture: the filters are off here, as in such frames)
+                fb = frame.FrameBuffers(S, lib=lib, alloc=frame.NumpyAlloc(), run_lf=False, run_cdef=False, run_lr=False,
+                                        band_rows=64 * int(rng.integers(1, 4)), compact=bool(rng.integers(0, 2)))
+                fb.run_bands()
+                ok, where = TI.planes_equal(S, exp, fb.output("p0"))
+                assert ok, ("bands", where)
                 kind = "intra"
             else:
                 mixed = rng.random() < 0.5
@@ -43,11 +49,9 @@ def main():
                               p_ii=float(rng.choice([0, 0.2])))
                 S = synth.make_inter_frame(rng, bpc, W, H, ssh, ssv, **kw)
                 exp = TF.oracle_frame(S)
-                has_intra = S.get("intra_tx") is not None and len(S["intra_tx"]) > 0
                 whole = -(-H // 64) * 64
-                variants = [dict(), dict(compact=True), dict(fused=True), dict(band_rows=whole, compact=True)]
-                if not has_intra:
-                    variants += [dict(band_rows=64 * int(rng.integers(1, 4)), compact=bool(rng.integers(0, 2)), fused=bool(rng.integers(0, 2)))]
+                variants = [dict(), dict(compact=True), dict(fused=True), dict(band_rows=whole, compact=True),
+                            dict(band_rows=64 * int(rng.integers(1, 4)), compact=bool(rng.integers(0, 2)), fused=bool(rng.integers(0, 2)))]
                 for v in variants:
                     fb = frame.FrameBuffers(S, lib=lib, alloc=frame.NumpyAlloc(), **v)
                     fb.run_bands() if v.get("band_rows") else fb.run()
